@@ -403,10 +403,40 @@ class Rig:
         return reduce_max_time(t, self.dev)
 
 
+DUMP_POOL = 148          # blocks the dump samples from: one per SM, fewer than any default batch holds, so the dump does not
+                         # depend on the batch size the free device memory allows
+DUMP_SAMPLE = 16         # archive blocks stored byte for byte
+DUMP_SEED = 20261020
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, d_out, ooff: np.ndarray, B: int):
+    """What the device-resident compress returned in its last step, as float arrays for comparing two builds: the archive size
+    of each of the first min(B, DUMP_POOL) blocks and the archive bytes of a fixed, seeded sample of them (with their indices).
+    Blocks are coded independently, so these do not depend on how many blocks the batch holds beyond the pool."""
+    pool = min(B, DUMP_POOL)
+    sizes = np.diff(ooff[:pool + 1].astype(np.int64))
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(pool, size=min(DUMP_SAMPLE, pool), replace=False))
+    budget = (DUMP_MAX_BYTES - 16 * pool) // 4             # float32 per archive byte; the two index arrays are float64
+    keep, total = [], 0
+    for i in pick:
+        if total + int(sizes[i]) > budget:
+            continue
+        keep.append(int(i))
+        total += int(sizes[i])
+    parts = [d_out[int(ooff[i]):int(ooff[i + 1])].cpu().numpy() for i in keep]
+    sample = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "archive_block_sizes.npy"), sizes.astype(np.float64))
+    np.save(os.path.join(out_dir, "archive_sample_blocks.npy"), np.asarray(keep, dtype=np.float64))
+    np.save(os.path.join(out_dir, "archive_sample_bytes.npy"), sample.astype(np.float32))
+
+
 def measure_config(rig: Rig, cfg_id: str, steps: int, warmup: int, batch_blocks: int = 0, sample_clocks: bool = False,
-                   timed_decompress_reps: int = 1, warm_host_path: bool = True):
+                   timed_decompress_reps: int = 1, warm_host_path: bool = True, dump_dir: str | None = None):
     """One config on this rank's GPU: device-resident compress (CUDA events), e2e compress and e2e decompress through the
-    host-buffer ABI (pinned buffers, copies inside the timed region), round trip checked."""
+    host-buffer ABI (pinned buffers, copies inside the timed region), round trip checked.  With `dump_dir`, rank 0 writes
+    what the last timed device-resident step returned (dump_outputs)."""
     import torch
     from tools import synth
     z, ctx, dev, world = rig.z, rig.ctx, rig.dev, rig.world
@@ -473,6 +503,8 @@ def measure_config(rig: Rig, cfg_id: str, steps: int, warmup: int, batch_blocks:
     t_dev = rig.max_time(e0.elapsed_time(e1) / 1e3)
     value = world * steps * in_bytes / 1e6 / t_dev
     ratio = float(ooff[B]) / in_bytes
+    if dump_dir and rig.rank == 0:
+        dump_outputs(dump_dir, d_out, ooff, B)
     del d_out
     del d_in
     torch.cuda.empty_cache()
@@ -688,7 +720,13 @@ def main():
     ap.add_argument("--no-library-multi-gpu", action="store_true")
     ap.add_argument("--all-configs", action="store_true", help="N > 1: also run the C1 .. C4 summary on every rank")
     ap.add_argument("--configs", default="C1,C2a,C2b,C2c,C3,C4,C5", help="which configs the summary holds (comma separated)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step computed to DIR/*.npy (a fixed, seeded sample of the archive)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -696,7 +734,7 @@ def main():
     rig = Rig()
     world, rank = rig.world, rig.rank
     head_id = args.config if args.config in CONFIGS else "C2a"
-    r = measure_config(rig, head_id, args.steps, args.warmup, args.batch_blocks, sample_clocks=True)
+    r = measure_config(rig, head_id, args.steps, args.warmup, args.batch_blocks, sample_clocks=True, dump_dir=args.dump_outputs)
     k_ms = r["kernel_ms"]
     achieved = r["A"] * r["in_bytes"] / (k_ms / 1e3) / 1e9
     traffic = None

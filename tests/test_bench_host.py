@@ -66,6 +66,37 @@ def test_algorithmic_bytes_of_the_survey():
     assert abs(bench.algorithmic_bytes(h1, 1 << 20, bench.BLOCK, 0.3, 0) - 66.3) < 0.5
 
 
+def test_dump_outputs_writes_a_fixed_sample_of_the_archive(tmp_path):
+    """--dump-outputs: float arrays only, within 64 MB, the same sample whatever the batch size beyond the pool."""
+    import numpy as np
+    import torch
+    import bench
+    rng = np.random.default_rng(7)
+    sizes = rng.integers(1, 5000, 400)
+    ooff = np.concatenate([[0], np.cumsum(sizes)]).astype(np.uint64)
+    arc = torch.from_numpy(rng.integers(0, 256, int(ooff[-1]), dtype=np.uint8))
+    bench.dump_outputs(str(tmp_path / "a"), arc, ooff, 400)
+    bench.dump_outputs(str(tmp_path / "b"), arc, ooff, 300)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["archive_block_sizes.npy", "archive_sample_blocks.npy", "archive_sample_bytes.npy"]
+    for f in files:
+        x, y = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, y)
+    got = np.load(tmp_path / "a" / "archive_sample_bytes.npy")
+    pick = np.load(tmp_path / "a" / "archive_sample_blocks.npy").astype(int)
+    assert len(pick) == bench.DUMP_SAMPLE
+    want = np.concatenate([arc.numpy()[int(ooff[i]):int(ooff[i + 1])] for i in pick])
+    assert np.array_equal(got, want.astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "a" / "archive_block_sizes.npy"), sizes[:bench.DUMP_POOL])
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= bench.DUMP_MAX_BYTES
+
+
+def test_bench_rejects_zero_steps_and_dump_on_the_reference_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert p.returncode == 2 and not p.stdout.strip(), p.stderr[-2000:]
+
+
 def test_c5_sweep_is_reduced_with_one_collective_and_survives_a_failed_rank():
     import bench
     rows = [{"seconds": 2.0, "out_bytes_per_gpu": 10 ** 9, "decompress_e2e_value": 0.0}, {"seconds": 4.0, "out_bytes_per_gpu": 10 ** 9, "decompress_e2e_value": 0.0}]
