@@ -43,6 +43,11 @@ namespace ZPAQSharp
         [DllImport(Lib)] public static extern long zpq_post_kind(int ph, int pm, byte* pcomp, ulong len);
         [DllImport(Lib)] public static extern long zpq_specialize_pcomp(int ph, int pm, byte* pcomp, ulong len, byte* source, ulong sourceCap, byte* log, ulong logCap);
         [DllImport(Lib)] public static extern int zpq_encoder_plan(byte* hdr, ulong hdrLen, uint smemBytes, uint blocksPerSm, int* out8);
+        [DllImport(Lib)] public static extern int zpq_scrypt(byte* pw, ulong pwLen, byte* salt, ulong saltLen, ulong n, uint r, uint p,
+            byte* output, ulong outLen);
+        [DllImport(Lib)] public static extern int zpq_stretch_key(byte* in32, byte* salt32, byte* out32);
+        [DllImport(Lib)] public static extern int zpq_aes_ctr(IntPtr ctx, byte* key, int keyLen, byte* iv8, byte* buf, ulong n, ulong offset);
+        [DllImport(Lib)] public static extern int zpq_aes_ctr_dev(IntPtr ctx, byte* key, int keyLen, byte* iv8, byte* dBuf, ulong n, ulong offset);
     }
 
     /// <summary>GPU-backed bodies for the LibZPAQ entry points of the compress/decompress path.</summary>
@@ -128,6 +133,57 @@ namespace ZPAQSharp
                     for (ulong i = 0; i < outOff[nb]; ++i) output.put(outBuf[i]);
                 }
             }
+        }
+
+        /// <summary>libzpaq stretchKey(out, in, salt), the body StretchKey.cs:13-163 restates: scrypt(in, 32, salt, 32,
+        /// 16384, 8, 1, out, 32), computed on the host by the library.  in32 is SHA-256 of the password.</summary>
+        public static void StretchKey(byte[] out32, byte[] in32, byte[] salt32)
+        {
+            if (out32 == null || in32 == null || salt32 == null || out32.Length < 32 || in32.Length < 32 || salt32.Length < 32)
+                LibZPAQ.error("stretchKey takes 32-byte buffers");
+            fixed (byte* po = out32, pi = in32, ps = salt32)
+                CheckHost(ZpaqB200Native.zpq_stretch_key(pi, ps, po));
+        }
+
+        /// <summary>libzpaq scrypt(pw, pwlen, salt, saltlen, n, r, p, buf, buflen) (RFC 7914), StretchKey.cs:13-163.</summary>
+        public static void Scrypt(byte[] pw, int pwlen, byte[] salt, int saltlen, int n, int r, int p, byte[] buf, int buflen)
+        {
+            if (pwlen < 0 || saltlen < 0 || buflen < 0 || r < 0 || p < 0 || n < 0) LibZPAQ.error("scrypt: negative argument");
+            fixed (byte* ppw = pw, ps = salt, pb = buf)
+                CheckHost(ZpaqB200Native.zpq_scrypt(ppw, (ulong)pwlen, ps, (ulong)saltlen, (ulong)n, (uint)r, (uint)p, pb, (ulong)buflen));
+        }
+
+        static void CheckHost(int rc)
+        {
+            if (rc != 0) LibZPAQ.error(Marshal.PtrToStringAnsi(ZpaqB200Native.zpq_last_error(IntPtr.Zero)));
+        }
+
+        internal static IntPtr Context() { return Ctx(); }
+        internal static void CheckCtx(int rc) { Check(rc); }
+    }
+
+    /// <summary>libzpaq 7.12's AES_CTR (the reference has it as prose only, LICENSE:635-665): AES in counter mode with
+    /// keystream block j = AES_key(iv[0..7] || big-endian j).  encrypt(buf, n, offset) XORs buf[0..n) with the keystream
+    /// from stream byte offset on the GPU; decrypting is the same call.  The key bytes are kept only to pass them to each
+    /// call; the library expands and wipes the key schedule inside the call.</summary>
+    public unsafe class AesCtrB200
+    {
+        readonly byte[] key;
+        readonly byte[] iv;
+
+        public AesCtrB200(byte[] key, int keylen, byte[] iv = null)
+        {
+            if (keylen != 16 && keylen != 24 && keylen != 32) LibZPAQ.error("AES_CTR: key length must be 16, 24 or 32");
+            this.key = new byte[keylen];
+            Array.Copy(key, this.key, keylen);
+            if (iv != null) { this.iv = new byte[8]; Array.Copy(iv, this.iv, 8); }
+        }
+
+        public void encrypt(byte[] buf, int n, ulong offset)
+        {
+            if (n < 0 || n > buf.Length) LibZPAQ.error("AES_CTR: n is outside the buffer");
+            fixed (byte* pk = key, pi = iv, pb = buf)
+                LibZPAQB200.CheckCtx(ZpaqB200Native.zpq_aes_ctr(LibZPAQB200.Context(), pk, key.Length, pi, pb, (ulong)n, offset));
         }
     }
     /// <summary>Replacement body of Compressor (Compressor.cs:12-304) over the batch ABI: same methods, same call order,

@@ -170,9 +170,36 @@ int zpq_decompress_blocks(zpq_ctx* ctx, const uint8_t* in, const uint64_t* in_of
  * the caller size `out`. */
 int64_t zpq_decompressed_bound(const uint8_t* in, const uint64_t* in_off, uint32_t nb);
 
+/* ---- encryption ---------------------------------------------------------------------------- */
+
+/* libzpaq 7.12's scrypt(pw, pwlen, salt, saltlen, n, r, p, out, outlen) (RFC 7914), which stretchKey calls
+ * (StretchKey.cs:13-163 restates it).  Host only, no context.  n must be a power of two >= 2, r >= 1, p >= 1
+ * (ZPQ_E_ARG otherwise); ZPQ_E_NOMEM when the 128 * r * n bytes of ROMix cannot be had.  outlen = 0 does nothing. */
+int zpq_scrypt(const uint8_t* pw, uint64_t pwlen, const uint8_t* salt, uint64_t saltlen, uint64_t n, uint32_t r, uint32_t p,
+               uint8_t* out, uint64_t outlen);
+
+/* libzpaq stretchKey(out32, in32, salt32), StretchKey.cs:13-163: scrypt(in32, 32, salt32, 32, 16384, 8, 1, out32, 32).
+ * As in libzpaq, in32 is SHA-256 of the password, computed by the caller.  Host only, no context. */
+int zpq_stretch_key(const uint8_t* in32, const uint8_t* salt32, uint8_t* out32);
+
+/* libzpaq AES_CTR(key, keylen, iv).encrypt(buf, n, offset) (the AES_CTR class of libzpaq 7.12; the reference has it as
+ * prose only, LICENSE:635-665), on the device, in place on a HOST buffer: buf[k] ^= byte (offset + k) % 16 of
+ * AES_key(iv[0..7] || big-endian 64-bit (offset + k) / 16).  iv8 may be NULL (8 zero bytes); keylen is 16, 24 or 32.
+ * Encryption and decryption are the same call.  A context over N devices gives each a contiguous byte range; every device
+ * works through at most 1 GiB of device memory at a time.  ZPQ_E_ARG for a bad key length, a NULL buffer with n > 0 or
+ * offset + n past 2^64 - 1; n = 0 does nothing.  No key material is kept after return. */
+int zpq_aes_ctr(zpq_ctx* ctx, const uint8_t* key, int keylen, const uint8_t* iv8, uint8_t* buf, uint64_t n, uint64_t offset);
+
+/* The same on a DEVICE buffer of device 0 of the context (no host<->device copy): enqueued on that device's stream (the
+ * context's own or the one zpq_set_stream gave) and completed before return, like zpq_compress_blocks_model_dev. */
+int zpq_aes_ctr_dev(zpq_ctx* ctx, const uint8_t* key, int keylen, const uint8_t* iv8, uint8_t* d_buf, uint64_t n,
+                    uint64_t offset);
+
 /* ---- introspection ------------------------------------------------------------------------- */
 
-/* Timing and launch statistics of the last compress/decompress call on device 0. */
+/* Timing and launch statistics of the last compress / decompress / AES call on device 0.  For zpq_aes_ctr and
+ * zpq_aes_ctr_dev: kernel_ms, h2d/d2h_ms and _bytes (host-buffer call; summed over its chunks), total_ms, launches, and
+ * kernel = "aes_ctr/128", "aes_ctr/192" or "aes_ctr/256"; the other fields are 0. */
 typedef struct zpq_stats {
   double h2d_ms, kernel_ms, d2h_ms, total_ms; /* CUDA-event times on the context's stream */
   double codec_kernel_ms;                      /* the coding kernel alone */

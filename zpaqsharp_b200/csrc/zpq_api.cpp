@@ -24,6 +24,7 @@
 #include <thread>
 
 #include "zpq_aot.h"
+#include "zpq_crypto.h"
 #include "zpq_device.h"
 #include "zpq_host.h"
 
@@ -1257,6 +1258,79 @@ int64_t copy_out(const std::string& s, char* out, uint64_t cap) {
   return (int64_t)s.size();
 }
 
+// ------------------------------------------------------------------------------------------
+// Encryption (libzpaq AES_CTR): the key schedule is expanded on the host and wiped when the call returns.
+// ------------------------------------------------------------------------------------------
+constexpr uint64_t kAesChunk = 1ull << 30;   // device bytes per device for a host-buffer call
+
+struct ScopedKey {
+  AesKey k;
+  ScopedKey(const uint8_t* key, int keylen) {
+    if (!key || (keylen != 16 && keylen != 24 && keylen != 32)) throw Failure(ZPQ_E_ARG, "AES key length must be 16, 24 or 32 bytes");
+    aes_expand_key(key, keylen, k);
+  }
+  ~ScopedKey() { secure_zero(&k, sizeof k); }
+  std::string name() const { return "aes_ctr/" + std::to_string(32 * (k.rounds - 6)); }
+};
+
+void check_aes_range(const uint8_t* buf, uint64_t n, uint64_t offset) {
+  if (!buf && n) throw Failure(ZPQ_E_ARG, "null buffer");
+  if (n && offset > ~0ull - n) throw Failure(ZPQ_E_ARG, "offset + n overflows the 64-bit stream position");
+}
+
+// Bytes [0, n) of a host buffer, stream offset `offset`, through one device in chunks of kAesChunk: copy in, kernel, copy
+// back.  A chunk lands at device address base + offset % 16, so its whole keystream blocks are 16-byte aligned.
+void aes_ctr_host_range(Device& d, const ScopedKey& key, const uint8_t* iv8, uint8_t* buf, uint64_t n, uint64_t offset) {
+  CU(cudaSetDevice(d.id));
+  cudaStream_t s = d.stream;
+  d.stats = zpq_stats{};
+  snprintf(d.stats.kernel, sizeof d.stats.kernel, "%s", key.name().c_str());
+  if (!n) return;
+  const uint64_t chunk = std::min<uint64_t>(n, kAesChunk);
+  reserve_io(d.in, chunk + 16, d.arena);
+  d.t_all.start(s);
+  for (uint64_t done = 0; done < n;) {
+    const uint64_t len = std::min<uint64_t>(n - done, kAesChunk), off = offset + done;
+    uint8_t* dev = d.in.as<uint8_t>() + off % 16;
+    d.t_h2d.start(s);
+    CU(cudaMemcpyAsync(dev, buf + done, len, cudaMemcpyHostToDevice, s));
+    d.t_h2d.stop(s);
+    d.t_kern.start(s);
+    CU(launch_aes_ctr(key.k, iv8, dev, len, off, s));
+    d.t_kern.stop(s);
+    d.t_d2h.start(s);
+    CU(cudaMemcpyAsync(buf + done, dev, len, cudaMemcpyDeviceToHost, s));
+    d.t_d2h.stop(s);
+    CU(cudaStreamSynchronize(s));
+    d.stats.h2d_ms += d.t_h2d.ms(); d.stats.kernel_ms += d.t_kern.ms(); d.stats.d2h_ms += d.t_d2h.ms();
+    d.stats.h2d_bytes += len; d.stats.d2h_bytes += len; d.stats.launches += 1;
+    done += len;
+  }
+  d.t_all.stop(s);
+  CU(cudaStreamSynchronize(s));
+  d.stats.total_ms = d.t_all.ms();
+}
+
+// Split [0, n) into one contiguous byte range per device; every range carries its own stream offset, so the devices never
+// exchange anything.
+void aes_ctr_host(zpq_ctx* ctx, const ScopedKey& key, const uint8_t* iv8, uint8_t* buf, uint64_t n, uint64_t offset) {
+  const size_t nd = ctx->devs.size();
+  if (nd == 1) { aes_ctr_host_range(ctx->devs[0], key, iv8, buf, n, offset); return; }
+  std::vector<std::string> errs(nd);
+  std::vector<int> codes(nd, 0);
+  std::vector<std::thread> th;
+  for (size_t k = 0; k < nd; ++k) {
+    const uint64_t lo = (uint64_t)((unsigned __int128)n * k / nd), hi = (uint64_t)((unsigned __int128)n * (k + 1) / nd);
+    th.emplace_back([&, k, lo, hi]() {
+      try { aes_ctr_host_range(ctx->devs[k], key, iv8, buf + lo, hi - lo, offset + lo); }
+      catch (const Failure& f) { codes[k] = f.code; errs[k] = f.what(); }
+      catch (const std::exception& e) { codes[k] = ZPQ_E_CUDA; errs[k] = e.what(); }
+    });
+  }
+  for (auto& t : th) t.join();
+  for (size_t k = 0; k < nd; ++k) if (codes[k]) throw Failure(codes[k], errs[k]);
+}
+
 }  // namespace
 
 // =========================================================================================
@@ -1607,6 +1681,47 @@ int zpq_get_stats(zpq_ctx* ctx, zpq_stats* out) {
   if (!ctx || !out) return ZPQ_E_ARG;
   *out = ctx->devs[0].stats;
   return ZPQ_OK;
+}
+
+int zpq_scrypt(const uint8_t* pw, uint64_t pwlen, const uint8_t* salt, uint64_t saltlen, uint64_t n, uint32_t r, uint32_t p,
+               uint8_t* out, uint64_t outlen) {
+  if ((!pw && pwlen) || (!salt && saltlen) || (!out && outlen)) return ZPQ_E_ARG;
+  return guarded(nullptr, [&]() { scrypt(pw, pwlen, salt, saltlen, n, r, p, out, outlen); });
+}
+
+int zpq_stretch_key(const uint8_t* in32, const uint8_t* salt32, uint8_t* out32) {
+  if (!in32 || !salt32 || !out32) return ZPQ_E_ARG;
+  return guarded(nullptr, [&]() { scrypt(in32, 32, salt32, 32, 16384, 8, 1, out32, 32); });
+}
+
+int zpq_aes_ctr(zpq_ctx* ctx, const uint8_t* key, int keylen, const uint8_t* iv8, uint8_t* buf, uint64_t n, uint64_t offset) {
+  if (!ctx) return ZPQ_E_ARG;
+  return guarded(ctx, [&]() {
+    check_aes_range(buf, n, offset);
+    const ScopedKey k(key, keylen);
+    aes_ctr_host(ctx, k, iv8, buf, n, offset);
+  });
+}
+
+int zpq_aes_ctr_dev(zpq_ctx* ctx, const uint8_t* key, int keylen, const uint8_t* iv8, uint8_t* d_buf, uint64_t n, uint64_t offset) {
+  if (!ctx) return ZPQ_E_ARG;
+  return guarded(ctx, [&]() {
+    check_aes_range(d_buf, n, offset);
+    const ScopedKey k(key, keylen);
+    Device& d = ctx->devs[0];
+    CU(cudaSetDevice(d.id));
+    cudaStream_t s = d.stream;
+    d.stats = zpq_stats{};
+    snprintf(d.stats.kernel, sizeof d.stats.kernel, "%s", k.name().c_str());
+    if (!n) return;
+    d.t_all.start(s);
+    d.t_kern.start(s);
+    CU(launch_aes_ctr(k.k, iv8, d_buf, n, offset, s));
+    d.t_kern.stop(s);
+    d.t_all.stop(s);
+    CU(cudaStreamSynchronize(s));
+    d.stats.kernel_ms = d.t_kern.ms(); d.stats.total_ms = d.t_all.ms(); d.stats.launches = 1;
+  });
 }
 
 }  // extern "C"

@@ -8,6 +8,10 @@ bytes reach the Writer in the reference's order and the archive is byte-identica
 the same calls.  `batch_blocks=1` codes every block when it ends.  The Decompresser decodes a wave of the blocks ahead of the
 one asked for in one call and serves `decompress(n)` from that.
 
+libzpaq's encryption pieces under their libzpaq names: `AES_CTR(key, iv, ctx).encrypt(buf, n, offset)` (the keystream
+computed and applied on the GPU), `stretchKey(in32, salt32)` and `scrypt(...)` (host), which StretchKey.cs:13-163 restates.
+As in libzpaq they are building blocks: the caller writes the salt and encrypts the archive bytes behind it.
+
 Deliberate limits of the device path, reported through `error()` like any other failure: one segment per block
 (the batch ABI codes independent blocks; SURVEY.md 8f lists multi-segment blocks as a later step).  Nothing here touches
 the oracle: without the CUDA library every call that needs the codec raises."""
@@ -510,3 +514,31 @@ class Decompresser:
 
     def buffered(self) -> int:                         # Decompresser.cs:201-204
         return len(self._arc) - self._pos
+
+
+# ---- encryption (libzpaq 7.12 AES_CTR, stretchKey, scrypt) --------------------------------------------------------------
+class AES_CTR:
+    """libzpaq AES_CTR(key, keylen, iv): encrypt(buf, n, offset) XORs buf[0..n) with the keystream from stream byte offset
+    (block j = AES(iv[0..7] || big-endian j)); decrypting is the same call.  key is 16, 24 or 32 bytes; iv 8 bytes or None."""
+
+    def __init__(self, key: bytes, iv: bytes | None = None, ctx: z.Context | None = None):
+        if len(key) not in (16, 24, 32):
+            error("AES key length must be 16, 24 or 32 bytes")
+        self._key, self._iv, self._ctx = bytes(key), iv, ctx
+
+    def encrypt(self, buf, n: int, offset: int):
+        """In place on the first n bytes of a writable buffer (bytearray, numpy uint8, ...)."""
+        a = buf if isinstance(buf, np.ndarray) else np.frombuffer(buf, dtype=np.uint8)
+        if n < 0 or n > a.size:
+            error("AES_CTR.encrypt: n is outside the buffer")
+        (self._ctx or z._ctx()).aes_ctr(a[:n], self._key, self._iv, offset)
+
+
+def stretchKey(in32: bytes, salt32: bytes) -> bytes:
+    """libzpaq stretchKey(out, in, salt): scrypt(in, salt, 16384, 8, 1, 32); in32 is SHA-256 of the password."""
+    return z.stretch_key(in32, salt32)
+
+
+def scrypt(pw: bytes, salt: bytes, n: int, r: int, p: int, dklen: int) -> bytes:
+    """libzpaq scrypt(pw, pwlen, salt, saltlen, n, r, p, out, outlen) (RFC 7914)."""
+    return z.scrypt(pw, salt, n, r, p, dklen)

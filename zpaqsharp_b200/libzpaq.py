@@ -28,6 +28,7 @@ ABI_SYMBOLS = [
     "zpq_device_state_bytes", "zpq_device_state_bytes_for", "zpq_compress_blocks", "zpq_compress_blocks_level", "zpq_compress_blocks_model",
     "zpq_compress_blocks_model_dev", "zpq_find_blocks", "zpq_decompress_blocks", "zpq_decompressed_bound",
     "zpq_get_stats", "zpq_version", "zpq_specialize_model", "zpq_encoder_plan", "zpq_post_kind", "zpq_specialize_pcomp",
+    "zpq_scrypt", "zpq_stretch_key", "zpq_aes_ctr", "zpq_aes_ctr_dev",
 ]
 
 
@@ -96,6 +97,10 @@ def load():
     L.zpq_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
     L.zpq_specialize_model.restype = C.c_int64
     L.zpq_specialize_model.argtypes = [u8p, C.c_uint64, C.c_char_p, C.c_uint64, C.c_char_p, C.c_uint64]
+    L.zpq_scrypt.argtypes = [u8p, C.c_uint64, u8p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, u8p, C.c_uint64]
+    L.zpq_stretch_key.argtypes = [u8p, u8p, u8p]
+    L.zpq_aes_ctr.argtypes = [C.c_void_p, u8p, C.c_int, u8p, u8p, C.c_uint64, C.c_uint64]
+    L.zpq_aes_ctr_dev.argtypes = [C.c_void_p, u8p, C.c_int, u8p, u8p, C.c_uint64, C.c_uint64]
     _lib = L
     return L
 
@@ -227,6 +232,34 @@ def find_blocks(archive) -> list:
     offs = np.zeros(2 * max(cnt, 1), dtype=np.uint64)
     L.zpq_find_blocks(p, n, offs.ctypes.data, cnt)
     return [(int(offs[2 * i]), int(offs[2 * i + 1])) for i in range(cnt)]
+
+
+# ---- key derivation (host, no device needed) ------------------------------------------------------
+def scrypt(pw: bytes, salt: bytes, n: int, r: int, p: int, dklen: int) -> bytes:
+    """libzpaq scrypt (RFC 7914), which stretchKey calls (StretchKey.cs:13-163)."""
+    out = C.create_string_buffer(max(dklen, 1))
+    rc = load().zpq_scrypt(bytes(pw), len(pw), bytes(salt), len(salt), n, r, p, out, dklen)
+    if rc != 0:
+        _raise(None, rc)
+    return out.raw[:dklen]
+
+
+def stretch_key(in32: bytes, salt32: bytes) -> bytes:
+    """libzpaq stretchKey (StretchKey.cs:13-163): scrypt(in32, salt32, 16384, 8, 1, 32); in32 is SHA-256 of the password."""
+    if len(in32) != 32 or len(salt32) != 32:
+        raise ZpaqError(E_ARG, "stretch_key takes 32-byte key and salt")
+    out = C.create_string_buffer(32)
+    rc = load().zpq_stretch_key(bytes(in32), bytes(salt32), out)
+    if rc != 0:
+        _raise(None, rc)
+    return out.raw
+
+
+def _aes_key_iv(key, iv):
+    key = bytes(key)
+    if iv is not None and len(iv) != 8:
+        raise ZpaqError(E_ARG, "the AES-CTR iv is 8 bytes")
+    return key, (bytes(iv) if iv is not None else None)
 
 
 def block_size_of(method: str) -> int:
@@ -361,6 +394,26 @@ class Context:
         if rc != 0:
             _raise(self._h, rc)
         return ooff
+
+    # -- encryption (libzpaq AES_CTR) --
+    def aes_ctr(self, buf, key: bytes, iv: bytes | None = None, offset: int = 0):
+        """AES_CTR(key, iv).encrypt(buf, len(buf), offset) on the GPU, in place on a writable buffer (bytearray, numpy uint8,
+        ...); returns buf.  Encrypting and decrypting are the same call."""
+        a = np.frombuffer(buf, dtype=np.uint8) if not isinstance(buf, np.ndarray) else buf
+        if a.dtype != np.uint8 or not a.flags.c_contiguous or not a.flags.writeable:
+            raise TypeError("aes_ctr works in place: pass a writable, contiguous uint8 buffer")
+        key, iv = _aes_key_iv(key, iv)
+        rc = load().zpq_aes_ctr(self._h, key, len(key), iv, a.ctypes.data if a.size else None, a.size, offset)
+        if rc != 0:
+            _raise(self._h, rc)
+        return buf
+
+    def aes_ctr_dev(self, d_ptr: int, n: int, key: bytes, iv: bytes | None = None, offset: int = 0):
+        """The same on n bytes at CUDA device address d_ptr (device 0 of the context), on the context's stream."""
+        key, iv = _aes_key_iv(key, iv)
+        rc = load().zpq_aes_ctr_dev(self._h, key, len(key), iv, C.c_void_p(d_ptr or None), n, offset)
+        if rc != 0:
+            _raise(self._h, rc)
 
     # -- decompression --
     def decompress_blocks(self, archive, offsets, out=None):
